@@ -582,6 +582,9 @@ def main():
     ap.add_argument("--integrated-threads", type=int, default=16,
                     help="worker threads of the plugin-linked ngmlr (16 = the GPU boxes' CPU quota measured best: "
                          "every thread blocks ~10 ms per SingleAlign batch, more threads only oversubscribe the CPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed device-resident path computed in its last step (the alignment of every "
+                         "interval, stage 0/2 candidates and scores) to DIR/<name>.npy, at most 64 MB in all")
     ap.add_argument("--integrated-reads", type=int, default=-1,
                     help="reads of the whole-ngmlr comparison (plain binary vs plugin-linked binary); "
                          "-1 = 2000 at N=1 on configs up to 100 Mb, else 0 (skipped)")
@@ -782,6 +785,8 @@ def main():
     sampler.mark_end()
     clocks = sampler.stop()
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, als, args.dp_only)
 
     # ---- (c) end to end from host buffers through the public calls: per step every context uploads its
     # reads ONCE (reads_upload), runs stage 0/2 on their sub-reads and brings candidates + scores back
@@ -976,6 +981,62 @@ def main():
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_BYTES = (64 << 20) - (1 << 16)   # 64 MB less room for the .npy headers
+ALIGN_FIELDS = ("ret", "Score", "Identity", "PositionOffset", "QStart", "QEnd", "NM", "alignmentLength", "cigarOpCount",
+                "svType")
+
+
+def dump_outputs(out_dir, als, dp_only):
+    """What a caller of the timed path receives after its last step, as float32 / float64 .npy files: every context's
+    alignments (fetch; one row per interval, contexts in order, CIGAR and MD text as CRC-32 and length) and stage 0/2
+    results (cs_fetch: per sub-read candidate ranges and best score, per candidate vote score, location, strand and
+    StrippedSW score). Per-candidate arrays that would exceed 64 MB in all are cut to a fixed, seeded sample of
+    candidates, whose indices are written as cs_sample.npy."""
+    import zlib
+    os.makedirs(out_dir, exist_ok=True)
+    al = {k: [] for k in ALIGN_FIELDS + ("first_position", "last_position", "cigar_crc32", "cigar_len", "md_crc32",
+                                         "md_len")}
+    cs = {k: [] for k in ("cs_start", "cs_max_score", "cs_vote_score", "cs_location", "cs_reverse", "cs_sw_score")}
+    base = 0
+    for a_ in als:
+        for r in a_.fetch():
+            for k in ALIGN_FIELDS:
+                al[k].append(getattr(r, k))
+            al["first_position"].append(r.firstPosition)
+            al["last_position"].append(r.lastPosition)
+            for k, t in (("cigar", r.pBuffer1), ("md", r.pBuffer2)):
+                b = t.encode() if isinstance(t, str) else bytes(t)
+                al[k + "_crc32"].append(zlib.crc32(b))
+                al[k + "_len"].append(len(b))
+        if not dp_only:
+            start, sc, lo, rv, sw, mx = a_.cs_fetch()
+            cs["cs_start"].append(start[:-1] + base)
+            base += int(start[-1])
+            for k, v in (("cs_max_score", mx), ("cs_vote_score", sc), ("cs_location", lo), ("cs_reverse", rv),
+                         ("cs_sw_score", sw)):
+                cs[k].append(v)
+    arrays = {"align_" + k: np.asarray(v, dtype=np.float32 if k in ("Score", "Identity") else np.float64)
+              for k, v in al.items()}
+    if not dp_only:
+        cs = {k: np.concatenate(v) for k, v in cs.items()}
+        cs["cs_start"] = np.append(cs["cs_start"], base)
+        for k in ("cs_start", "cs_location"):
+            arrays[k] = cs[k].astype(np.float64)
+        for k in ("cs_max_score", "cs_vote_score", "cs_reverse", "cs_sw_score"):
+            arrays[k] = cs[k].astype(np.float32)
+        per_cand = ("cs_vote_score", "cs_location", "cs_reverse", "cs_sw_score")
+        fixed = sum(v.nbytes for k, v in arrays.items() if k not in per_cand)
+        row = sum(arrays[k].itemsize for k in per_cand)
+        keep = max(0, (DUMP_BYTES - fixed) // (row + 8))
+        if base > keep:
+            idx = np.sort(np.random.default_rng(0).choice(base, size=keep, replace=False))
+            for k in per_cand:
+                arrays[k] = arrays[k][idx]
+            arrays["cs_sample"] = idx.astype(np.float64)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def parity_check(wl, cpu_aligned, gpu_first, gpu_cs, st02, n_stage02_reads):

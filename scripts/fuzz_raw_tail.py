@@ -12,8 +12,9 @@ with the oracle's rule 2 on inputs built to hit the corner: corridors 13-48 colu
 row is "tail"), scorings with cheap gap opens / expensive mismatches, short periodic sequences that tie a lot.
 Prints the number of cells and mismatches; exits non-zero on any mismatch."""
 import argparse
-import sys
+import hashlib
 import os
+import sys
 
 import numpy as np
 
@@ -25,23 +26,15 @@ SCORINGS = [(1.0, -20.0, -1.0, -1.0, -1.0, 0.15), (2.0, -8.0, -1.0, -2.0, -0.5, 
             (3.0, -30.0, -2.0, -1.0, -1.0, 0.0), (1.0, -1.0, -1.0, -1.0, -1.0, 0.15), (2.0, -5.0, -5.0, -5.0, -1.0, 0.15)]
 
 
-def main():
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--cells", type=float, default=1.2e8)
-    ap.add_argument("--seed", type=int, default=1)
-    args = ap.parse_args()
+def problems(seed, max_cells):
+    """The seeded fuzz inputs: (scoring, ref, qry, offsets, lengths, cells), 200 per scoring in turn, until
+    `max_cells` cells are reached."""
     from ngmlr_b200 import corridor, synth
-    from oracle_lib import Oracle, Reference
-    rng = np.random.default_rng(args.seed)
-    orc = Oracle()
+    rng = np.random.default_rng(seed)
     cells = 0
-    bad = 0
     n = 0
-    per_scoring = {}
-    n_scalar_probe = n_scalar_differs = 0
-    while cells < args.cells:
+    while cells < max_cells:
         sc = SCORINGS[n % len(SCORINGS)]
-        ref_eng = Reference(scoring=sc)
         for _ in range(200):
             H = int(rng.integers(20, 400))
             W = int(rng.integers(13, 49))
@@ -56,25 +49,67 @@ def main():
             shift = int(rng.integers(-5, 15))
             o, l = corridor.corridor_linear(len(q), W)
             o = (o + 10 + shift).astype(np.int32)
-            a = ref_eng.fill(r.tobytes(), q.tobytes(), o, l, 0)
-            b = orc.fill(r.tobytes(), q.tobytes(), o, l, sc, 2)
-            if n_scalar_probe < 3000:   # how often does this input separate the SSE semantics from the scalar rule at all?
-                n_scalar_probe += 1
-                s1 = orc.fill(r.tobytes(), q.tobytes(), o, l, sc, 1)
-                n_scalar_differs += not (np.array_equal(a[0], s1[0]) and a[1:] == s1[1:])
-            same = (np.array_equal(a[0], b[0]) and np.float32(a[1]).view(np.uint32) == np.float32(b[1]).view(np.uint32)
-                    and a[2:] == b[2:])
             c = int(np.maximum(np.minimum(o + l, len(r)) - np.maximum(o, 0), 0).sum())
             cells += c
-            per_scoring[sc] = per_scoring.get(sc, 0) + c
-            if not same:
-                bad += 1
-                print("MISMATCH", sc, H, W, a[1:], b[1:], file=sys.stderr)
-        ref_eng.close()
+            yield sc, r.tobytes(), q.tobytes(), o, l, c
         n += 1
+
+
+def fill_digest(res):
+    """Directions, best score bits and best cell of one fill, as stored by --golden files."""
+    dirs, bs, bx, by = res
+    h = hashlib.sha256(np.ascontiguousarray(dirs).tobytes())
+    h.update(np.array([np.float32(bs).view(np.uint32), bx, by], dtype=np.int64).tobytes())
+    return h.hexdigest()[:16]
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--cells", type=float, default=1.2e8)
+    ap.add_argument("--seed", type=int, default=1)
+    ap.add_argument("--golden", default=None,
+                    help="JSON file with the reference's fill digests for --cells / --seed (tests/golden/"
+                         "compiled_ref_golden.json, section raw_tail): compare with those instead of the compiled "
+                         "reference")
+    args = ap.parse_args()
+    from oracle_lib import Oracle, Reference
+    orc = Oracle()
+    golden = None
+    if args.golden:
+        import json
+        golden = json.load(open(args.golden))["raw_tail"]
+        assert golden["cells"] == args.cells and golden["seed"] == args.seed, "golden file is for another run"
+        golden = golden["fills"]
+    engines = {}
+    cells = 0
+    bad = 0
+    n = 0
+    per_scoring = {}
+    n_scalar_probe = n_scalar_differs = 0
+    for sc, r, q, o, l, c in problems(args.seed, args.cells):
+        if golden is not None:
+            want = golden[n]
+        else:
+            if sc not in engines:
+                engines[sc] = Reference(scoring=sc)
+            want = fill_digest(engines[sc].fill(r, q, o, l, 0))
+        b = orc.fill(r, q, o, l, sc, 2)
+        if n_scalar_probe < 3000:   # how often does this input separate the SSE semantics from the scalar rule at all?
+            n_scalar_probe += 1
+            n_scalar_differs += fill_digest(orc.fill(r, q, o, l, sc, 1)) != want
+        cells += c
+        per_scoring[sc] = per_scoring.get(sc, 0) + c
+        if fill_digest(b) != want:
+            bad += 1
+            print("MISMATCH", sc, len(q), int(l[0]), b[1:], file=sys.stderr)
+        n += 1
+    for e in engines.values():
+        e.close()
+    if golden is not None:
+        assert n == len(golden), "golden file is for another run"
     print(f"{n_scalar_differs} of the first {n_scalar_probe} problems separate the as-coded SSE semantics from the pure "
           f"scalar rule (the fuzz is not vacuous)")
-    print(f"cells {cells} problems {n * 200} mismatches {bad}; cells per scoring: "
+    print(f"cells {cells} problems {n} mismatches {bad}; cells per scoring: "
           + ", ".join(f"{k}: {v}" for k, v in per_scoring.items()))
     sys.exit(1 if bad else 0)
 

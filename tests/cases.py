@@ -126,3 +126,33 @@ def corridor_cases(seed=33, n=48):
                         realign=int(rng.integers(0, 2)), multiplier=int(rng.choice([1, 1, 2, 4])),
                         anchors=anchors, on_ref_start=on_ref_start, ext_qstart=ext_qs, full_len=full_len))
     return out
+
+
+def corridor_fuzz_cases(seed=21, n=60):
+    """Seeded inputs of the corridor builders compared with the compiled reference (test_host_logic): dicts with
+    q, r, corridor, on_ref_start, ext_qstart, full_len, anchors [(onRead, onRef, isReverse)], their (x, y) form
+    ax / ay, multiplier, and the four arguments a, b, c, d of estimateCorridor(a, a + b, c, c + d)."""
+    rng = np.random.default_rng(seed)
+    out = []
+    for _ in range(n):
+        q = int(rng.integers(1, 6000))
+        r = int(max(1, q + rng.integers(-q // 3 - 1, q // 3 + 2)))
+        cor = int(rng.choice([40, 400, 1600, 3333, 8192]))
+        # anchored corridor: forward and reverse anchors (mapping to (x, y) as at src/AlignmentBuffer.cpp:149-158)
+        on_ref_start = int(rng.integers(1000, 10**9))
+        ext_qs = int(rng.integers(0, 50))
+        full_len = q + ext_qs + int(rng.integers(0, 300))
+        anchors, ax, ay = [], [], []
+        for _a in range(int(rng.integers(0, 12))):
+            on_read = int(rng.integers(0, q + 1)) + ext_qs
+            on_ref = on_ref_start + int(rng.integers(0, r + 1))
+            rev = int(rng.integers(0, 2))
+            anchors.append((on_read, on_ref, rev))
+            ax.append(on_ref - on_ref_start)
+            ay.append(full_len - on_read - 256 - ext_qs if rev else on_read - ext_qs)
+        mult = int(rng.choice([1, 1, 2, 4]))
+        a, b = int(rng.integers(0, 50000)), int(rng.integers(0, 50000))
+        c, d = int(rng.integers(0, 10**9)), int(rng.integers(0, 60000))
+        out.append(dict(q=q, r=r, corridor=cor, on_ref_start=on_ref_start, ext_qstart=ext_qs, full_len=full_len,
+                        anchors=anchors, ax=ax, ay=ay, multiplier=mult, a=a, b=b, c=c, d=d))
+    return out

@@ -72,11 +72,8 @@ def test_no_cpu_fallback():
     assert lib.CreateAlignment(0) is None  # plugin factory fails loudly too
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference headers not present")
-def test_compat_header_layout_equals_reference_header():
-    """sizeof/offsetof of Align, CorridorLine, PositionNM, Interval and the vtable slot order of
-    IAlignment in include/ngmlr_b200_ialignment.h == src/IAlignment.h."""
-    probe = r'''
+# sizeof/offsetof of Align, CorridorLine, PositionNM, Interval and the vtable slot order of IAlignment
+PROBE = r'''
 #include <stdio.h>
 #include <stddef.h>
 #include HEADER
@@ -102,14 +99,17 @@ int main() {
   printf("\n");
   return 0;
 }'''
+
+
+def test_compat_header_layout_equals_reference_header():
+    """The PROBE numbers of include/ngmlr_b200_ialignment.h == those of the reference's src/IAlignment.h
+    (tests/golden/compiled_ref_golden.json, written by tests/golden/make_ref_golden.py)."""
     import tempfile
-    outs = []
+    import golden_util as gu
     with tempfile.TemporaryDirectory() as d:
-        for hdr, inc in (('"IAlignment.h"', "/root/reference/src"),
-                         ('"ngmlr_b200_ialignment.h"', os.path.join(ROOT, "include"))):
-            path = os.path.join(d, "p.cpp")
-            open(path, "w").write(probe.replace("HEADER", hdr))
-            subprocess.run(["g++", "-std=c++11", "-w", "-I", inc, "-o", os.path.join(d, "p"), path,
-                            "-Wl,--unresolved-symbols=ignore-all"], check=True)
-            outs.append(subprocess.run([os.path.join(d, "p")], capture_output=True, text=True, check=True).stdout)
-    assert outs[0] == outs[1], outs
+        path = os.path.join(d, "p.cpp")
+        open(path, "w").write(PROBE.replace("HEADER", '"ngmlr_b200_ialignment.h"'))
+        subprocess.run(["g++", "-std=c++11", "-w", "-I", os.path.join(ROOT, "include"), "-o", os.path.join(d, "p"), path,
+                        "-Wl,--unresolved-symbols=ignore-all"], check=True)
+        got = subprocess.run([os.path.join(d, "p")], capture_output=True, text=True, check=True).stdout
+    assert got == gu.load("compiled_ref_golden.json")["abi_layout"]

@@ -1,12 +1,12 @@
 """CPU tests of the candidate-search row: the C restatement (oracle/cs_oracle.c) and the numpy
-builder of the reference-format index (ngmlr_b200/refindex.py) against the WHOLE unmodified
-reference (oracle/_ref/libngmlr_full.so: SequenceProvider, CompactPrefixTable, CS) when present,
-and against each other always."""
+builder of the reference-format index (ngmlr_b200/refindex.py) against what the WHOLE unmodified
+reference (oracle/_ref/libngmlr_full.so: SequenceProvider, CompactPrefixTable, CS) returned, and
+against each other."""
 import numpy as np
 import pytest
 
 import cs_cases
-from oracle_lib import CsOracle, CsReference
+from oracle_lib import CsOracle
 
 
 @pytest.fixture(scope="module")
@@ -51,40 +51,32 @@ def test_oracle_search_basic_properties(contigs, cs_oracle):
 
 
 @pytest.fixture(scope="module")
-def whole_ref(contigs, tmp_path_factory):
-    """The unmodified reference initialised on the test genome (its singletons: once per process)."""
-    if not CsReference.available():
-        pytest.skip("oracle/_ref/libngmlr_full.so not built")
-    path = str(tmp_path_factory.mktemp("cs") / "ref.fa")
-    with open(path, "w") as f:
-        for i, c in enumerate(contigs):
-            f.write(f">c{i}\n{c.tobytes().decode()}\n")
-    return CsReference(path)
+def whole_ref():
+    """What the unmodified reference, initialised on the test genome, returned (tests/golden/compiled_ref_golden.json,
+    written by tests/golden/make_ref_golden.py)."""
+    import golden_util as gu
+    return gu.load("compiled_ref_golden.json")
 
 
 def test_oracle_equals_whole_reference(contigs, cs_oracle, whole_ref):
-    ref = whole_ref
-    assert ref.concat_len == cs_oracle.concat_len and ref.ref_starts() == cs_oracle.ref_starts()
-    a, b = ref.index(), cs_oracle.index()
-    for x, y in zip(a, b):
-        assert np.array_equal(x, y)
-    for sub in cs_cases.subreads(250, 17, contigs):
-        if len(sub) == 0:
-            continue
-        for bits in (16, 8):   # table size must not matter (overflow -> retry with a larger table)
-            assert ref.search(sub, table_bits=bits) == cs_oracle.search(sub)
-    for p in (0, 1, 999, 1000, 1001, 5555, 61000, ref.concat_len - 100, ref.concat_len - 1, ref.concat_len):
-        assert ref.decode(p) == cs_oracle.decode(p)
-    # DecodeRefSequenceExact (alignment windows, corridor 0 as in extractReferenceSequenceForAlignment)
-    from ngmlr_b200 import refindex
-    enc = refindex.encode_reference(contigs)
-    wins = cs_cases.exact_windows(enc.ref_start, enc.ref_len)
-    assert len(wins) > 500
-    for st, ln in wins:
-        assert ref.decode_exact(st, ln) == cs_oracle.decode_exact(st, ln), (st, ln)
-    assert ref.decode_exact(ref.concat_len, 10) is None and cs_oracle.decode_exact(ref.concat_len, 10) is None
-    for st, ln, c in ((5000, 100, 12), (5001, 101, 12), (61000, 64, 40)):   # non-zero corridor as well
-        assert ref.decode_exact(st, ln, c) == cs_oracle.decode_exact(st, ln, c)
+    import golden_util as gu
+    ref = whole_ref["whole_reference"]
+    assert ref["concat_len"] == cs_oracle.concat_len and ref["ref_starts"] == cs_oracle.ref_starts()
+    assert gu.digest(*cs_oracle.index()) == ref["index_sha"]
+    subs = [s for s in cs_cases.subreads(250, 17, contigs) if len(s)]
+    assert len(subs) == len(ref["search"])
+    for sub, (sha, mh) in zip(subs, ref["search"]):
+        got, got_mh = cs_oracle.search(sub)
+        assert gu.digest(np.array([x[0] for x in got], np.float32), np.array([x[1] for x in got], np.uint64),
+                         np.array([x[2] for x in got], np.int32)) == sha and got_mh == mh
+    for p, sha in ref["decode"]:
+        d = cs_oracle.decode(p)
+        assert (None if d is None else gu.digest(d)) == sha, p
+    # DecodeRefSequenceExact (alignment windows, corridor 0 as in extractReferenceSequenceForAlignment): the
+    # reference's windows are those of decode_exact_golden.json (test_oracle_decode_exact_matches_golden)
+    assert cs_oracle.decode_exact(cs_oracle.concat_len, 10) is None
+    for st, ln, c, sha in ref["decode_exact_corridor"]:   # non-zero corridor as well
+        assert gu.digest(cs_oracle.decode_exact(st, ln, c)) == sha
 
 
 def test_oracle_decode_exact_matches_golden(contigs, cs_oracle):
@@ -136,52 +128,32 @@ def test_cache_files_round_trip(contigs, tmp_path, built):
         ngmfiles.c_read_index(str(tmp_path / "sig.ngm"))
 
 
-@pytest.mark.skipif(not CsReference.available(), reason="oracle/_ref/libngmlr_full.so not built")
-def test_cache_files_are_byte_compatible_with_the_reference(contigs, tmp_path, built):
-    """The UNMODIFIED reference writes <fasta>-enc.2.ngm and <fasta>-ht-13-2.2.ngm (in a subprocess:
-    its singletons initialise once per process); ngmfiles reads them into the arrays refindex builds,
-    and writes the same bytes (the index file entirely; the encoded reference up to the end of the used
-    part of binRef -- the reference writes its uninitialised allocation tail)."""
-    import subprocess
-    import sys
-    from ngmlr_b200 import ngmfiles, refindex
-    fasta = str(tmp_path / "ref.fa")
-    with open(fasta, "w") as f:
-        for i, c in enumerate(contigs):
-            f.write(f">contig{i} some description\n{c.tobytes().decode()}\n")
-    code = ("import ctypes, sys; lib = ctypes.CDLL(sys.argv[1]); "
-            "sys.exit(lib.ref_cs_init_save(sys.argv[2].encode()))")
-    run = subprocess.run([sys.executable, "-c", code, CsReference.PATH, fasta], capture_output=True, text=True,
-                         timeout=600)
-    assert run.returncode == 0, run.stderr[-2000:]
-    enc_path, idx_path = fasta + "-enc.2.ngm", fasta + "-ht-13-2.2.ngm"
+def test_cache_files_are_byte_compatible_with_the_reference(contigs, tmp_path, built, whole_ref):
+    """The UNMODIFIED reference writes <fasta>-enc.2.ngm and <fasta>-ht-13-2.2.ngm for the test genome (contig names
+    with a description); ngmfiles and the library's C writers write the same bytes (the index file entirely; the
+    encoded reference up to the end of the used part of binRef -- the reference writes its uninitialised allocation
+    tail): digests of the reference's files are stored."""
+    import golden_util as gu
+    from ngmlr_b200 import ngmfiles
+    gold = whole_ref["cache_files"]
     ref, idx = built
-    got_ref, names = ngmfiles.read_encoded_reference(enc_path)
-    assert np.array_equal(got_ref.enc, ref.enc) and got_ref.concat_len == ref.concat_len
-    assert got_ref.ref_start == ref.ref_start and got_ref.ref_len == ref.ref_len
+    names = gold["names"]
     assert names == [f"contig{i}" for i in range(len(contigs)) if contigs[i].size > 10]
-    got_idx, skip, off = ngmfiles.read_index(idx_path)
-    assert (got_idx.k, skip, off) == (13, 2, 0)
-    assert np.array_equal(got_idx.tab, idx.tab) and np.array_equal(got_idx.rci, idx.rci)
-    assert np.array_equal(got_idx.pos, idx.pos)
     # writers: same bytes
     ngmfiles.write_index(str(tmp_path / "mine-ht.ngm"), idx)
-    assert open(tmp_path / "mine-ht.ngm", "rb").read() == open(idx_path, "rb").read()
+    assert gu.digest(open(tmp_path / "mine-ht.ngm", "rb").read()) == gold["index_sha"]
     skipped = [int(c.size) for c in contigs if not c.size > 10]
     ngmfiles.write_encoded_reference(str(tmp_path / "mine-enc.ngm"), ref, names, skipped_lens=skipped)
-    mine, theirs = open(tmp_path / "mine-enc.ngm", "rb").read(), open(enc_path, "rb").read()
+    mine = open(tmp_path / "mine-enc.ngm", "rb").read()
     defined = 24 + 128 * len(ref.ref_start) + int(ref.enc.size)
-    assert len(mine) == len(theirs) and mine[:defined] == theirs[:defined]
-    # ... and the library's C writers / readers on the reference's own files
+    assert len(mine) == gold["enc_len"] and gu.digest(mine[:defined]) == gold["enc_defined_sha"]
+    # ... and the library's C writers
     ngmfiles.c_write_index(str(tmp_path / "c-ht.ngm"), idx)
-    assert open(tmp_path / "c-ht.ngm", "rb").read() == open(idx_path, "rb").read()
+    assert gu.digest(open(tmp_path / "c-ht.ngm", "rb").read()) == gold["index_sha"]
     ngmfiles.c_write_encoded_reference(str(tmp_path / "c-enc.ngm"), ref, names, skipped_lens=skipped)
     assert open(tmp_path / "c-enc.ngm", "rb").read() == mine
-    c_ref, c_names = ngmfiles.c_read_encoded_reference(enc_path)
+    c_ref, c_names = ngmfiles.c_read_encoded_reference(str(tmp_path / "mine-enc.ngm"))
     assert np.array_equal(c_ref.enc, ref.enc) and c_ref.ref_start == ref.ref_start and c_names == names
-    c_idx, c_skip, c_off = ngmfiles.c_read_index(idx_path)
-    assert (c_idx.k, c_skip, c_off) == (13, 2, 0) and np.array_equal(c_idx.tab, idx.tab)
-    assert np.array_equal(c_idx.rci, idx.rci) and np.array_equal(c_idx.pos, idx.pos)
 
 
 class _OracleBackend:
@@ -243,38 +215,23 @@ def _interval_tasks(contigs, enc):
 def test_batched_compute_alignment_equals_the_reference(contigs, cs_oracle, whole_ref, oracle):
     """ngmlr_b200.intervals.compute_alignments (window extraction, corridor per attempt, retry policy)
     with the oracle as its backend == AlignmentBuffer::computeAlignment of the unmodified reference."""
-    import ctypes as C
+    import golden_util as gu
     from ngmlr_b200 import refindex
     from ngmlr_b200.intervals import compute_alignments
-    lib = whole_ref.lib
-    if not hasattr(lib, "ref_compute_alignment"):
-        pytest.skip("libngmlr_full.so predates ref_compute_alignment")
     enc = refindex.encode_reference(contigs)
     tasks = _interval_tasks(contigs, enc)
+    want = whole_ref["whole_reference"]["compute_alignment"]
+    assert len(want) == len(tasks)
     got, calls = compute_alignments(_OracleBackend(cs_oracle, oracle), tasks)
     n_valid = n_retry = 0
-    for t, g, nc in zip(tasks, got, calls):
-        n = len(t.anchors)
-        a0 = (C.c_int * max(n, 1))(*[a[0] for a in t.anchors])
-        a1 = (C.c_ulonglong * max(n, 1))(*[a[1] for a in t.anchors])
-        a2 = (C.c_int * max(n, 1))(*[a[2] for a in t.anchors])
-        ints = (C.c_int * 12)()
-        fl = (C.c_float * 2)()
-        cap = 8 * len(t.read_seq) + 64
-        cig, md = C.create_string_buffer(cap), C.create_string_buffer(cap)
-        ok = lib.ref_compute_alignment(C.c_ulonglong(t.on_ref_start), C.c_ulonglong(t.on_ref_stop), n, a0, a1, a2,
-                                       t.corridor, t.read_seq, t.ext_qstart, t.ext_qend, t.full_read_length,
-                                       int(t.realign), int(t.full_alignment), int(t.short_read), ints, fl,
-                                       cig, cap, md, cap, None, 0)
-        assert bool(ok) == (g is not None), (t.corridor, nc)
+    for t, g, nc, w in zip(tasks, got, calls, want):
+        assert (w is not None) == (g is not None), (t.corridor, nc)
         if g is None:
             continue
         n_valid += 1
         n_retry += nc > 1
-        assert cig.value.decode() == g["cigar"] and md.value.decode() == g["md"]
-        assert (ints[1], ints[2], ints[3], ints[4], ints[5]) == (g["qstart"], g["qend"], g["nm"],
-                                                                  g["alignment_length"], g["cigar_op_count"])
-        assert ints[11] == g["position_offset"]
-        assert np.float32(fl[0]).view(np.uint32) == np.uint32(g["score_bits"])
-        assert np.float32(fl[1]).view(np.uint32) == np.uint32(g["identity_bits"])
+        assert w["cigar_sha"] == gu.digest(g["cigar"]) and w["md_sha"] == gu.digest(g["md"])
+        for k in ("qstart", "qend", "nm", "alignment_length", "cigar_op_count", "position_offset", "score_bits",
+                  "identity_bits"):
+            assert w[k] == g[k], k
     assert n_valid >= 24 and n_retry >= 3, (n_valid, n_retry)

@@ -173,73 +173,26 @@ def test_text_stage_fast_paths_equal_column_by_column_version():
         assert ints[11] * 3 == len(w_pos) and list(nm[:len(w_pos)]) == w_pos, case
 
 
-def _ref_full_lib():
-    import ctypes as C
-    from oracle_lib import CsReference
-    if not CsReference.available():
-        pytest.skip("oracle/_ref/libngmlr_full.so not built")
-    lib = C.CDLL(CsReference.PATH)
-    if not hasattr(lib, "ref_corridor"):
-        pytest.skip("libngmlr_full.so predates the corridor entry points")
-    return lib, C
-
-
-def _ref_corridor(lib, C, kind, qry_len, ref_len, corridor_arg, realign=0, anchors=(), on_ref_start=0,
-                  ext_qstart=0, read_part_len=256, full_read_len=0):
-    n = len(anchors)
-    on_read = (C.c_int * max(n, 1))(*[a[0] for a in anchors])
-    on_ref = (C.c_ulonglong * max(n, 1))(*[a[1] for a in anchors])
-    rev = (C.c_int * max(n, 1))(*[a[2] for a in anchors])
-    off = np.zeros(max(qry_len, 1), dtype=np.int32)
-    ln = np.zeros(max(qry_len, 1), dtype=np.int32)
-    h = lib.ref_corridor(kind, qry_len, ref_len, corridor_arg, realign, n, on_read, on_ref, rev,
-                         C.c_ulonglong(on_ref_start), ext_qstart, read_part_len, full_read_len,
-                         off.ctypes.data_as(C.c_void_p), ln.ctypes.data_as(C.c_void_p))
-    assert h == qry_len
-    return off[:h], ln[:h]
-
-
 def test_corridor_builders_equal_the_compiled_reference():
     """corridor.py (float32 numpy) against the reference's own getCorridorLinear / getCorridorFull /
     getCorridorEndpoints / AlignmentBuffer::getCorridorEndpointsWithAnchors / estimateCorridor
-    (src/AlignmentBuffer.cpp:68-197, 1454-1467), called through oracle/ref_cs_shim.cpp."""
-    import pytest as _pt  # noqa: F401
-    lib, C = _ref_full_lib()
-    lib.ref_estimate_corridor.argtypes = [C.c_int, C.c_int, C.c_longlong, C.c_longlong]
-    rng = np.random.default_rng(21)
-    for _ in range(60):
-        q = int(rng.integers(1, 6000))
-        r = int(max(1, q + rng.integers(-q // 3 - 1, q // 3 + 2)))
-        cor = int(rng.choice([40, 400, 1600, 3333, 8192]))
-        o, l = _ref_corridor(lib, C, 0, q, r, cor)
-        eo, el = corridor.corridor_linear(q, cor)
-        assert np.array_equal(o, eo) and np.array_equal(l, el)
-        o, l = _ref_corridor(lib, C, 1, q, r, r)      # getCorridorFull is called with the reference length
-        eo, el = corridor.corridor_full(q, r)
-        assert np.array_equal(o, eo) and np.array_equal(l, el)
+    (src/AlignmentBuffer.cpp:68-197, 1454-1467): digests of what they returned through oracle/ref_cs_shim.cpp
+    (tests/golden/compiled_ref_golden.json, written by tests/golden/make_ref_golden.py)."""
+    import cases
+    import golden_util as gu
+    gold = gu.load("compiled_ref_golden.json")["corridor"]
+    cs = cases.corridor_fuzz_cases()
+    assert len(gold) == len(cs)
+    for c, g in zip(cs, gold):
+        q, r, cor = c["q"], c["r"], c["corridor"]
+        assert gu.digest(*corridor.corridor_linear(q, cor)) == g["linear"]
+        assert gu.digest(*corridor.corridor_full(q, r)) == g["full"]
         for realign in (0, 1):
-            o, l = _ref_corridor(lib, C, 2, q, r, cor, realign)
             eo, el = corridor.corridor_endpoints(q, r, cor, realign=bool(realign))
-            assert np.array_equal(o, eo) and np.array_equal(l, el), (q, r, cor, realign)
-        # anchored corridor: forward and reverse anchors (mapping to (x, y) as at :149-158)
-        on_ref_start = int(rng.integers(1000, 10**9))
-        ext_qs = int(rng.integers(0, 50))
-        full_len = q + ext_qs + int(rng.integers(0, 300))
-        anchors, ax, ay = [], [], []
-        for _a in range(int(rng.integers(0, 12))):
-            on_read = int(rng.integers(0, q + 1)) + ext_qs
-            on_ref = on_ref_start + int(rng.integers(0, r + 1))
-            rev = int(rng.integers(0, 2))
-            anchors.append((on_read, on_ref, rev))
-            ax.append(on_ref - on_ref_start)
-            ay.append(full_len - on_read - 256 - ext_qs if rev else on_read - ext_qs)
-        mult = int(rng.choice([1, 1, 2, 4]))
-        o, l = _ref_corridor(lib, C, 3, q, r, mult, 0, anchors, on_ref_start, ext_qs, 256, full_len)
-        eo, el = corridor.corridor_endpoints_with_anchors(q, r, ax, ay, mult)
-        assert np.array_equal(o, eo) and np.array_equal(l, el), (q, r, anchors, mult)
-        a, b = int(rng.integers(0, 50000)), int(rng.integers(0, 50000))
-        c, d = int(rng.integers(0, 10**9)), int(rng.integers(0, 60000))
-        assert lib.ref_estimate_corridor(a, a + b, c, c + d) == corridor.estimate_corridor(b, d)
+            assert gu.digest(eo, el) == g["endpoints"][realign], (q, r, cor, realign)
+        eo, el = corridor.corridor_endpoints_with_anchors(q, r, c["ax"], c["ay"], c["multiplier"])
+        assert gu.digest(eo, el) == g["anchors"], (q, r, c["anchors"], c["multiplier"])
+        assert corridor.estimate_corridor(c["b"], c["d"]) == g["estimate"]
 
 
 def test_corridor_builders_match_golden():

@@ -1,11 +1,13 @@
-"""CPU tests: the oracle restatement against (a) the committed golden vectors produced by the
-unmodified reference and (b) the compiled reference itself when it is present (this container)."""
+"""CPU tests: the oracle restatement against the committed golden vectors produced by the unmodified
+reference (tests/golden/make_golden.py, tests/golden/make_ref_golden.py)."""
 import numpy as np
 import pytest
 
 import cases
 import golden_util as gu
-from oracle_lib import DEFAULT_SCORING, Reference, same_alignment
+from oracle_lib import DEFAULT_SCORING
+
+REF_GOLD = gu.load("compiled_ref_golden.json")   # tests/golden/make_ref_golden.py
 
 
 @pytest.mark.parametrize("setname", ["default", "weird", "mild"])
@@ -68,24 +70,19 @@ def test_oracle_cells_formula(oracle):
     assert oracle.cells(len(p.ref), p.offsets, p.lengths) == int(np.maximum(hi - lo, 0).sum()) == p.cells
 
 
-@pytest.mark.skipif(not Reference.available(), reason="oracle/_ref not built (no /root/reference here)")
 @pytest.mark.parametrize("sc,seed", [(DEFAULT_SCORING, 21), (cases.WEIRD_SCORING, 22), (cases.MILD_SCORING, 23)])
 def test_oracle_vs_compiled_reference(oracle, sc, seed):
-    ref = Reference(sc)
-    try:
-        for p in cases.random_problems(10, seed, max_len=900):
-            a = ref.single_align(p.ref, p.qry, p.offsets, p.lengths, p.ext_qstart, p.ext_qend)
-            b = oracle.single_align(p.ref, p.qry, p.offsets, p.lengths, p.ext_qstart, p.ext_qend,
-                                    scoring=sc, rule=0)
-            assert same_alignment(a, b) == []
-            da = ref.fill(p.ref, p.qry, p.offsets, p.lengths, 0)
-            db = oracle.fill(p.ref, p.qry, p.offsets, p.lengths, sc, 0)
-            assert np.array_equal(da[0], db[0]) and da[1:] == db[1:]
-        refs, qrys = cases.sw_pairs(64, seed)
-        for r, q in zip(refs, qrys):
-            assert ref.ssw_score(r, q) == oracle.ssw_score(r, q) == oracle.ssw_score(r, q, striped=True)
-    finally:
-        ref.close()
+    gold = REF_GOLD["convex"][str(seed)]
+    for i, (p, rec) in enumerate(zip(cases.random_problems(10, seed, max_len=900), gold["records"])):
+        assert gu.digest(p.ref, p.qry, p.offsets, p.lengths) == rec["input_sha"], "generator drifted"
+        b = oracle.single_align(p.ref, p.qry, p.offsets, p.lengths, p.ext_qstart, p.ext_qend, scoring=sc, rule=0)
+        gu.check_against_record(b, rec, f"{seed}[{i}]")
+        assert b["score_bits"] == rec["score_bits"]
+        db = oracle.fill(p.ref, p.qry, p.offsets, p.lengths, sc, 0)
+        assert gu.digest(db[0]) == rec["dirs_sha"] and [int(np.float32(db[1]).view(np.uint32)), *db[2:]] == rec["best"]
+    refs, qrys = cases.sw_pairs(64, seed)
+    for r, q, want in zip(refs, qrys, gold["sw"]):
+        assert want == oracle.ssw_score(r, q) == oracle.ssw_score(r, q, striped=True)
 
 
 def test_oracle_score_select_matches_golden(oracle):
@@ -104,32 +101,30 @@ def test_oracle_score_select_matches_golden(oracle):
             assert list(order) == g["order"]
 
 
-@pytest.mark.skipif(not Reference.available(), reason="compiled reference absent (GPU box / no /root/reference)")
 def test_oracle_score_select_vs_compiled_reference(oracle):
-    from oracle_lib import CsReference, score_select_cases
-    if not CsReference.available():
-        pytest.skip("libngmlr_full.so absent")
-    for sc in score_select_cases(5, 1500):
-        if sc.size == 0:
-            continue
+    from oracle_lib import score_select_cases
+    gold = REF_GOLD["score_select"]
+    scs = [sc for sc in score_select_cases(5, 1500) if sc.size]
+    assert len(scs) == len(gold["kept"])
+    orders = []
+    for sc, k, m in zip(scs, gold["kept"], gold["mq"]):
         o = oracle.score_select(sc)
-        r = CsReference.score_select(sc)
-        assert o[1:] == r[1:] and np.array_equal(o[0], r[0])
+        assert o[1:] == (k, m)
+        orders.append(o[0])
+    assert gu.digest(np.concatenate(orders)) == gold["order_sha"]
 
 
 def test_raw_tail_corner_fuzz_against_the_compiled_reference():
     """scripts/fuzz_raw_tail.py (DESIGN.md section 2): the compiled reference's fill vs the single-pass rule 2
     the CUDA RAW kernel implements, on inputs built to hit the tail-cell best-tracking corner (narrow
     corridors, scorings outside the default class). The full run (1.2e8 cells, 0 mismatches) is recorded in
-    DESIGN.md; this is its quick version."""
+    DESIGN.md; this is its quick version, against the reference's fills stored for it."""
     import os
     import subprocess
     import sys
-    from oracle_lib import Reference
-    if not Reference.available():
-        pytest.skip("oracle/_ref/libngmlr_ref.so not built")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, os.path.join(root, "scripts", "fuzz_raw_tail.py"), "--cells", "4e6", "--seed", "3"],
+    r = subprocess.run([sys.executable, os.path.join(root, "scripts", "fuzz_raw_tail.py"), "--cells", "4e6", "--seed", "3",
+                        "--golden", os.path.join(root, "tests", "golden", "compiled_ref_golden.json")],
                        capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-500:] + r.stderr[-500:]
     assert "mismatches 0" in r.stdout and "not vacuous" in r.stdout

@@ -1,37 +1,33 @@
 """The real call stream of plain ngmlr -- every IAlignment::SingleAlign / BatchScore / SingleScore call the
 unmodified reference makes on a FASTQ, recorded by the decorators of oracle/record_aligners.cpp
-(oracle/_ref/ngmlr_rec; SURVEY.md section 7 step 0) -- replayed call by call:
+(oracle/_ref/ngmlr_rec; SURVEY.md section 7 step 0) with what the reference returned, stored as a sample --
+replayed call by call:
   * CPU: through the oracle (pins the C restatement on retries x5, realignments, full matrices,
     corridors several thousand columns wide -- inputs the seeded generators only approximate);
   * GPU (-m gpu): through the CUDA library (batched convex path with the device text stage, sub-read
     scorer), bit for bit against what the reference returned."""
-import json
+import lzma
 import os
-import subprocess
 import sys
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REC = os.path.join(ROOT, "oracle", "_ref", "ngmlr_rec")
 sys.path.insert(0, os.path.join(ROOT, "scripts"))
-
-needs_rec = pytest.mark.skipif(not os.path.exists(REC), reason="oracle/_ref/ngmlr_rec not built")
 
 
 @pytest.fixture(scope="module")
 def stream(tmp_path_factory):
-    d = str(tmp_path_factory.mktemp("rec"))
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "record_workload.py"), "--reads", "28",
-                        "--genome-mb", "1", "--contigs", "2", "--threads", "8", "--median", "5000", "--sv",
-                        "--seed", "7", "--out", d], capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stderr[-2000:]
+    """A sample of the call stream (tests/golden/recorded_calls.bin.xz, written by tests/golden/make_ref_golden.py
+    from `scripts/record_workload.py --reads 28 --genome-mb 1 --contigs 2 --threads 8 --median 5000 --sv --seed 7`)."""
+    path = str(tmp_path_factory.mktemp("rec") / "calls.bin")
+    with lzma.open(os.path.join(ROOT, "tests", "golden", "recorded_calls.bin.xz")) as f, open(path, "wb") as out:
+        out.write(f.read())
     from replay_workload import parse
-    aligns, pairs = parse(os.path.join(d, "calls.bin"))
-    side = json.load(open(os.path.join(d, "calls.json")))
+    aligns, pairs = parse(path)
     assert len(aligns) >= 40 and len(pairs) >= 1000
-    return aligns, pairs, side
+    return aligns, pairs
 
 
 def _same(a, r):
@@ -42,9 +38,8 @@ def _same(a, r):
             and r["qstart"] == a["qstart"] and r["qend"] == a["qend"])
 
 
-@needs_rec
 def test_oracle_equals_the_reference_on_its_real_call_stream(stream, oracle):
-    aligns, pairs, _side = stream
+    aligns, pairs = stream
     bad = [i for i, a in enumerate(aligns)
            if not _same(a, oracle.single_align(a["ref"], a["qry"], a["off"], a["len"], a["qs"], a["qe"]))]
     assert not bad, bad[:5]
@@ -55,11 +50,10 @@ def test_oracle_equals_the_reference_on_its_real_call_stream(stream, oracle):
         assert int(np.float32(oracle.ssw_score(r, q)).view(np.uint32)) == sb
 
 
-@needs_rec
 @pytest.mark.gpu
 def test_cuda_library_equals_the_reference_on_its_real_call_stream(stream):
     from ngmlr_b200 import B200Aligner, PackedBatch
-    aligns, pairs, _side = stream
+    aligns, pairs = stream
     al = B200Aligner(0)
     try:
         for on_device in (True, False):

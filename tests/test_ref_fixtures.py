@@ -1,8 +1,8 @@
 """The reference's own test fixtures (test/data/test_2, test_4, test_5, test_6 with their expected
 files, copied as data to tests/golden/ref_fixtures/; the checks of test/test_*.sh restated without
 samtools / bedtools): BASELINE.json configs[0] verbatim.
-  * CPU: the unmodified reference binary (oracle/_ref/ngmlr) reproduces expected.bed / expected.txt --
-    which validates the restated checks themselves;
+  * CPU: what the unmodified reference binary (oracle/_ref/ngmlr) wrote for them (stored) reproduces
+    expected.bed / expected.txt -- which validates the restated checks themselves;
   * GPU (-m gpu): the same binary with its aligners swapped for the CUDA plugin (oracle/_ref/ngmlr_b200)
     passes the same checks and writes the same SAM records as the plain binary.
 FASTA reads are converted to FASTQ (constant quality 'I'): the reference overflows a 2-byte quality buffer
@@ -76,33 +76,44 @@ def _bed(records):
     return out
 
 
-def _checks(exe, tmp):
-    # (test_1 -- read names longer than the parser's limit -- is not reproduced by the reference's own HEAD,
-    # which cuts names at 250 characters where expected.txt still holds 277; it concerns the FASTA parser only)
+# (fixture, reference, reads, options) of the checks of test/test_*.sh.
+# (test_1 -- read names longer than the parser's limit -- is not reproduced by the reference's own HEAD,
+# which cuts names at 250 characters where expected.txt still holds 277; it concerns the FASTA parser only)
+FIXTURE_RUNS = [("test_2", "ref_chr21_20kb.fa", "reads_100_2200bp.fa", ()),
+                ("test_4", "reference.fasta.gz", "read.fa.gz", ("-x", "pacbio", "-t", "4")),
+                ("test_5", "reference.fasta.gz", "read.fa.gz", ("-x", "pacbio", "-t", "4")),
+                ("test_6", "reference.fasta.gz", "read.fa.gz", ("-x", "pacbio", "-t", "4"))]
+
+
+def _checks(records):
+    """records: fixture -> SAM records (lists of columns) of one binary on it."""
     # test_2: simple read lengths -> expected.bed
-    recs2 = _run(exe, tmp, "test_2", "ref_chr21_20kb.fa", "reads_100_2200bp.fa")
-    assert _bed(recs2) == open(os.path.join(FIX, "test_2", "expected.bed")).read().splitlines()
+    assert _bed(records["test_2"]) == open(os.path.join(FIX, "test_2", "expected.bed")).read().splitlines()
     # test_4: primary alignment, columns 1-5 sorted
-    recs4 = _run(exe, tmp, "test_4", "reference.fasta.gz", "read.fa.gz", ("-x", "pacbio", "-t", "4"))
-    got = sorted("\t".join(r[:5]) for r in recs4)
+    got = sorted("\t".join(r[:5]) for r in records["test_4"])
     assert got == open(os.path.join(FIX, "test_4", "expected.txt")).read().splitlines()
     # test_5: max query name length (<= 254 characters of names); test_6: five reads -> five records
-    recs5 = _run(exe, tmp, "test_5", "reference.fasta.gz", "read.fa.gz", ("-x", "pacbio", "-t", "4"))
-    assert sum(len(r[0]) + 1 for r in recs5) <= 254
-    recs6 = _run(exe, tmp, "test_6", "reference.fasta.gz", "read.fa.gz", ("-x", "pacbio", "-t", "4"))
-    assert len(recs6) == 5   # samtools view -Sc
-    return dict(t2=recs2, t4=recs4, t5=recs5, t6=recs6)
+    assert sum(len(r[0]) + 1 for r in records["test_5"]) <= 254
+    assert len(records["test_6"]) == 5   # samtools view -Sc
 
 
-@pytest.mark.skipif(not os.path.exists(PLAIN), reason="oracle/_ref/ngmlr not built")
-def test_plain_reference_passes_its_own_fixture_checks(tmp_path):
-    _checks(PLAIN, str(tmp_path))
+def _run_all(exe, tmp):
+    return {t: _run(exe, tmp, t, ref, reads, extra) for t, ref, reads, extra in FIXTURE_RUNS}
+
+
+def test_plain_reference_passes_its_own_fixture_checks():
+    """Columns 1-6 of what plain ngmlr wrote for the fixtures (tests/golden/compiled_ref_golden.json, written by
+    tests/golden/make_ref_golden.py) pass the restated checks."""
+    import golden_util as gu
+    _checks(gu.load("compiled_ref_golden.json")["fixture_records"])
 
 
 @pytest.mark.gpu
 @pytest.mark.skipif(not (os.path.exists(PLAIN) and os.path.exists(SWAPPED)), reason="oracle/_ref binaries not built")
 def test_plugin_linked_ngmlr_passes_the_reference_fixture_checks(tmp_path):
-    a = _checks(SWAPPED, str(tmp_path))
-    b = _checks(PLAIN, str(tmp_path))
+    a = _run_all(SWAPPED, str(tmp_path))
+    b = _run_all(PLAIN, str(tmp_path))
+    _checks(a)
+    _checks(b)
     for k in a:
         assert sorted(map(tuple, a[k])) == sorted(map(tuple, b[k])), k   # every SAM column, every record
